@@ -3,6 +3,7 @@
 pairs/sec on 3DMatch-size clouds).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--pairs B] [--config C]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (pyramid -> KPConv encoder -> cross-encoder -> regressor ->
 Kabsch) over one batch of B synthetic 3DMatch-shaped pairs per GPU.  Default workload: BASELINE
@@ -11,6 +12,10 @@ config 2 (one ~20k-point pair, batch 1, 1 GPU).  N>1 (torchrun): every rank runs
 
 Prints ONE JSON line on rank 0 (see the keys in `main`).  Timing: CUDA events per step on the
 launching stream, W >= 3 warm-up steps, L2 flushed between timed steps, max over ranks.
+
+--dump-outputs DIR writes the output dict of the last timed step (rank 0's pairs) as DIR/<name>.npy.  The
+inputs and weights come from fixed seeds, so two builds run with the same arguments can be compared output by
+output.
 """
 from __future__ import annotations
 
@@ -31,6 +36,11 @@ import torch  # noqa: E402
 
 WEIGHT_SEED = 2024
 POOL = 8          # distinct synthetic pairs rotated through the steps
+DUMP_BYTES = 64 * 10 ** 6     # --dump-outputs writes at most this much
+# the reference's output dict; per-cloud entries are lists (one tensor per pair) with the points on this axis
+OUTPUT_KEYS = ('src_feat_un', 'tgt_feat_un', 'src_feat', 'tgt_feat', 'src_kp', 'tgt_kp', 'src_kp_warped',
+               'tgt_kp_warped', 'src_overlap', 'tgt_overlap', 'pose')
+POINT_AXIS = {'feat_un': 0, 'kp': 0, 'feat': 1, 'kp_warped': 1, 'overlap': 1}
 _T0 = time.time()
 
 
@@ -60,6 +70,8 @@ def parse():
     ap.add_argument('--inflight', type=int, default=10,
                     help='independent pairs in flight per GPU (CUDA-graph executors on private streams); 1 = serial')
     ap.add_argument('--graph', type=int, default=1, help='1: CUDA-graph executor (GraphedRegTR); 0: eager forward')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB)')
     return ap.parse_args()
 
 
@@ -135,6 +147,44 @@ class ClockSampler:
                 'samples': len(sm), 'reasons': sorted(reasons)}
 
 
+def dump_outputs(out, folder):
+    """Write one forward's output dict as <folder>/<name>.npy: per-cloud entries as <key>_<pair>, floating point as
+    float32 (anything else as float64).  Above DUMP_BYTES the per-cloud arrays keep a seeded sample of their points,
+    the same rows for every array of a cloud, written beside them as <side>_sample_rows_<pair>.  Returns
+    (bytes written, whether the points were sampled)."""
+    items = []                                  # (file name, (side, pair) or None, points axis, tensor)
+    for key in OUTPUT_KEYS:
+        val = out[key]
+        if torch.is_tensor(val):
+            items.append((key, None, None, val))
+        else:
+            side, kind = key.split('_', 1)
+            items += [(f'{key}_{b}', (side, b), POINT_AXIS[kind], t) for b, t in enumerate(val)]
+    arrays = {}
+    for name, _, _, t in items:
+        t = t.detach().cpu()
+        arrays[name] = (t.float() if t.is_floating_point() else t.double()).numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    fixed = sum(arrays[name].nbytes for name, cloud, _, _ in items if cloud is None)
+    rows = {}
+    if total > DUMP_BYTES:
+        keep = 0.99 * (DUMP_BYTES - fixed) / (total - fixed)     # 1 %: room for the row lists
+        for name, cloud, axis, _ in items:
+            if cloud is None:
+                continue
+            if cloud not in rows:
+                n = arrays[name].shape[axis]
+                rng = np.random.default_rng([('src', 'tgt').index(cloud[0]), cloud[1]])
+                rows[cloud] = np.sort(rng.choice(n, size=min(n, max(1, int(n * keep))), replace=False))
+            arrays[name] = np.take(arrays[name], rows[cloud], axis=axis)
+        for (side, b), r in rows.items():
+            arrays[f'{side}_sample_rows_{b}'] = r.astype(np.float64)
+    os.makedirs(folder, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(folder, name + '.npy'), np.ascontiguousarray(a))
+    return sum(a.nbytes for a in arrays.values()), bool(rows)
+
+
 # ------------------------------------------------------------------------- CPU baseline
 
 def cpu_forward_fn(cfg, sd):
@@ -149,7 +199,7 @@ def cpu_forward_fn(cfg, sd):
                 meta = pre.preprocess_refcpp(cfg, [src, tgt], ref)
             else:
                 meta = pre.preprocess(cfg, [src, tgt])
-            return regtr_oracle.forward(sd, cfg, [src], [tgt], meta=meta)['pose']
+            return regtr_oracle.forward(sd, cfg, [src], [tgt], meta=meta)
     return run, ('reference C++ core (oracle/_ref: nanoflann + grid_subsampling)' if ref is not None
                  else 'oracle C restatement (brute-force first-K)')
 
@@ -195,17 +245,20 @@ def run_reference(args, rank, world):
     log(f'reference arm: {cores} threads of {os.cpu_count()} cores')
     for i in range(max(args.warmup, 1)):
         run(*pool[i % len(pool)])
-    # each step = a bounded sample of the workload: ONE pair (the workload has B*N pairs/step); the run is
-    # additionally bounded in time (REGTR_REF_BUDGET_S, default 120 s) so that large K still ends in minutes
-    budget = float(os.environ.get('REGTR_REF_BUDGET_S', 120))
+    # each step = a bounded sample of the workload: ONE pair (the workload has B*N pairs/step).  All --steps steps
+    # run; REGTR_REF_BUDGET_S=<seconds> opts in to stopping early (after >= 3 steps) once that much time has passed,
+    # and `executed_steps` then reports how many ran
+    budget = float(os.environ.get('REGTR_REF_BUDGET_S', 'inf'))
     t0 = time.perf_counter()
     done = 0
     for i in range(args.steps):
-        run(*pool[i % len(pool)])
+        last = run(*pool[i % len(pool)])
         done += 1
         if done >= 3 and time.perf_counter() - t0 > budget:
             break
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        log('outputs of the last step: %d bytes, points sampled: %s' % dump_outputs(last, args.dump_outputs))
     v = done / dt
     line = dict(metric='pairs/sec on 3DMatch-size clouds (~20k pts); pose err vs ref', value=v, unit='pairs/s',
                 n_gpus=args.gpus, steps=args.steps, warmup=args.warmup, ms_per_step=1000 * dt / done,
@@ -447,9 +500,11 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}                                   # output dict of the last timed step (--dump-outputs)
+
     def device_step(step):
         batch, _ = batch_at(step, resident)
-        out = runner(batch)
+        out = last['out'] = runner(batch)
         return gather_poses(out['pose'], B * world) if world > 1 else out['pose']
 
     def e2e_step(step):
@@ -493,7 +548,9 @@ def main():
         host_rec['blocked_on_gpu_ms_per_step'] = 1e3 * waited / K            # of which: waiting in event.synchronize
         host_rec['host_work_ms_per_step'] = 1e3 * (t_cpu - waited) / K       # Python + CUDA API calls
         log(f'submit loop {1e3 * t_cpu / K:.3f} ms/step, of which waiting for the GPU {1e3 * waited / K:.3f}')
-        outs += [o['host_pose'].clone() for o in pipe.drain()]
+        drained = pipe.drain()                  # oldest first: the last one is the last step's
+        outs += [o['host_pose'].clone() for o in drained]
+        last['out'] = drained[-1]
         pipe.join()
         if world > 1:                           # the run's poses, gathered over the ranks (288 B / pair)
             gather_poses(torch.cat(outs, dim=1).to(dev, non_blocking=True), B * K * world)
@@ -522,6 +579,8 @@ def main():
         barrier()
     launches = ops.LAUNCHES - launches0
     log(f'device-resident: {t_dev_ms / K:.3f} ms/step')
+    if args.dump_outputs and rank == 0:        # before the next forwards reuse the graphs' output buffers
+        log('outputs of the last timed step: %d bytes, points sampled: %s' % dump_outputs(last['out'], args.dump_outputs))
 
     # ---------------- end-to-end: host buffers in, pose on the host out
     h2d = sum(host[j][0].numel() * 4 + host[j][1].numel() * 4 for j in batch_at(W, host)[1])

@@ -1,6 +1,8 @@
-"""Seeded synthetic inputs of the metric fixtures (shared by make_golden.py and tests/test_eval.py):
-Redwood-format ground-truth scenes, perturbed estimates, ModelNet-style batches."""
+"""Seeded synthetic inputs of the fixtures (shared by make_golden.py and the tests): Redwood-format ground-truth
+scenes, perturbed estimates, ModelNet-style batches, loss inputs, 3DMatch-layout pair files, sequences for the
+padding helpers and the clouds of the C++ pre-processing cross-check."""
 import os
+import pickle
 
 import numpy as np
 
@@ -114,3 +116,39 @@ def grad_sample_index(name, numel, k=32):
     import zlib
     rng = np.random.default_rng(zlib.crc32(name.encode()))
     return np.sort(rng.choice(numel, size=min(k, numel), replace=False))
+
+
+def write_pair_files(folder, n_pairs=11, seed=0):
+    """A small dataset in the 3DMatch layout: `<folder>/test/scene/cloud_bin_<i>.pth` (float64 ndarrays, like the
+    real files) and `<folder>/info.pkl`; returns the info dict."""
+    import torch
+    rng = np.random.default_rng(seed)
+    infos = dict(rot=[], trans=[], src=[], tgt=[], overlap=[])
+    os.makedirs(os.path.join(folder, 'test', 'scene'), exist_ok=True)
+    for i in range(n_pairs + 1):
+        pts = rng.normal(size=(int(rng.integers(50, 400)), 3))
+        torch.save(pts, os.path.join(folder, 'test', 'scene', f'cloud_bin_{i}.pth'))
+    for i in range(n_pairs):
+        q, _ = np.linalg.qr(rng.normal(size=(3, 3)))
+        infos['rot'].append(q); infos['trans'].append(rng.normal(size=(3, 1)))
+        infos['src'].append(f'test/scene/cloud_bin_{i + 1}.pth'); infos['tgt'].append(f'test/scene/cloud_bin_{i}.pth')
+        infos['overlap'].append(float(rng.uniform(0.1, 0.9)))
+    with open(os.path.join(folder, 'info.pkl'), 'wb') as f:
+        pickle.dump(infos, f)
+    return infos
+
+
+def seq_inputs(seed=2):
+    """Ragged (N, 5) sequences for pad_sequence / unpad_sequences / split_src_tgt, and a padded (6, 11, 4, 5) stack."""
+    import torch
+    rng = np.random.default_rng(seed)
+    seqs = [torch.from_numpy(rng.normal(size=(n, 5)).astype(np.float32)) for n in (7, 3, 11, 1)]
+    six = torch.from_numpy(rng.normal(size=(6, 11, 4, 5)).astype(np.float32))
+    return seqs, six
+
+
+def refcpp_inputs(seed=9):
+    """Two clouds (400 + 500 points) for the radius-search / grid-subsampling cross-check of the C++ core."""
+    rng = np.random.default_rng(seed)
+    pts = rng.uniform(-0.5, 0.5, size=(900, 3)).astype(np.float32)
+    return pts, np.array([400, 500])

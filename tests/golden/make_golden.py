@@ -2,7 +2,8 @@
 
 Run in the build container only (needs /root/reference):
 
-    python tests/golden/make_golden.py
+    make -C oracle ref                      # refcpp_fixture binds the reference's C++ core (oracle/_ref)
+    python tests/golden/make_golden.py      # every fixture; `... make_golden.py data`: data.npz + refcpp.npz
 
 Every fixture is produced by the reference's own modules, imported through
 oracle/ref_bridge.py (third-party stubs per SURVEY.md Appendix A), on seeded
@@ -395,6 +396,78 @@ def grad_fixture():
     print('grad: parameters with a gradient', n, 'total loss', float(fx['loss_total']))
 
 
+def _ref_module(rel):
+    """One reference source file imported on its own (its package __init__ pulls in h5py and friends)."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location('ref_' + os.path.basename(rel)[:-3], os.path.join(ref_bridge.REF_SRC, rel))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+def data_fixture():
+    """Input side (tests/test_data.py): the reference's `collate_pair` on three items of the seeded pair files, its
+    sequence helpers on seeded sequences, the full 3DMatch benchmark pickle (`test_3DMatch_info.pkl`, every row) and
+    the SHA-256 of the shipped sample clouds, whose fp32 values the real_*_input.npz fixtures hold."""
+    import pickle
+    import tempfile
+    import eval_inputs as ei
+    from regtr_b200 import data as D
+    collate = _ref_module(os.path.join('data_loaders', 'collate_functions.py')).collate_pair
+    R = _ref_module(os.path.join('utils', 'seq_manipulation.py'))
+    fx = {}
+    with tempfile.TemporaryDirectory() as tmp:
+        ei.write_pair_files(tmp)
+        ds = D.ThreeDMatchPairs(tmp, os.path.join(tmp, 'info.pkl'))
+        out = collate([ds[i] for i in (4, 0, 7)])
+    fx['collate_keys'] = np.array(list(out))
+    for k, v in out.items():
+        if torch.is_tensor(v):
+            fx[f'collate|{k}'] = _np(v)
+        else:
+            for b, x in enumerate(v):
+                fx[f'collate|{k}|{b}'] = _np(x) if torch.is_tensor(x) else np.array(x)
+    seqs, six = ei.seq_inputs()
+    for i, kw in enumerate((dict(), dict(require_padding_mask=True, require_lens=True))):
+        padded, mask, lens = R.pad_sequence(seqs, **kw)
+        fx[f'pad{i}_padded'] = _np(padded)
+        if mask is not None:
+            fx[f'pad{i}_mask'] = _np(mask)
+        if lens is not None:
+            fx[f'pad{i}_lens'] = np.array(lens)
+    lens = [s.shape[0] for s in seqs]
+    for b, x in enumerate(R.unpad_sequences(six, lens)):
+        fx[f'unpad_{b}'] = _np(x)
+    src, tgt = R.split_src_tgt(torch.cat(seqs), lens)
+    for b, x in enumerate(list(src) + list(tgt)):
+        fx[f'split_{b}'] = _np(x)
+    info = pickle.load(open(os.path.join(ref_bridge.REF_SRC, 'datasets', '3dmatch', 'test_3DMatch_info.pkl'), 'rb'))
+    fx.update(info_rot=np.stack(info['rot']), info_trans=np.stack(info['trans']), info_src=np.array(info['src']),
+              info_tgt=np.array(info['tgt']), info_overlap=np.array(info['overlap'], dtype=np.float64))
+    for case, (_, _, src_rel, tgt_rel) in REAL_CASES.items():
+        if src_rel.startswith('indoor/'):
+            for rel in (src_rel, tgt_rel):
+                fx[f'cloud_sha256|{rel}'] = sha(torch.load(os.path.join(REF_DATA, rel), weights_only=False))
+    np.savez_compressed(os.path.join(OUT, 'data.npz'), **fx)
+    print('data', len(fx), 'arrays;', len(info['rot']), 'benchmark rows')
+
+
+def refcpp_fixture():
+    """The reference's C++ pre-processing core (nanoflann radius search, hash-map grid subsampling; built into
+    oracle/_ref by `make -C oracle ref`) on the clouds of eval_inputs.refcpp_inputs: every query's in-radius
+    neighbours in the order returned (ragged: counts + concatenated ids) and the subsampled level sizes."""
+    import eval_inputs as ei
+    from oracle import pre
+    ref = pre.RefCpp()
+    pts, lens = ei.refcpp_inputs()
+    b = ref.batch_neighbors(pts, pts, lens, lens, 0.11, 64)
+    valid = b < len(pts)
+    _, len_r = ref.batch_subsample(pts, lens, 0.1)
+    np.savez_compressed(os.path.join(OUT, 'refcpp.npz'), neighbor_counts=valid.sum(1).astype(np.int32),
+                        neighbor_ids=b[valid].astype(np.int32), subsample_lens=len_r)
+    print('refcpp', int(valid.sum()), 'neighbours; level sizes', len_r.tolist())
+
+
 if __name__ == '__main__':
     torch.manual_seed(0)
     np.random.seed(0)
@@ -409,6 +482,12 @@ if __name__ == '__main__':
     if len(sys.argv) > 1 and sys.argv[1] == 'grad':
         grad_fixture()
         sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == 'data':
+        data_fixture()
+        refcpp_fixture()
+        sys.exit(0)
+    data_fixture()
+    refcpp_fixture()
     eval_fixtures()
     loss_fixture()
     grad_fixture()

@@ -1,5 +1,6 @@
 """CPU tests of the input pipeline (SURVEY.md 8f N2, regtr_b200/data.py): file formats of the reference's
-3DMatch loader, collate layout, size bucketing, read-ahead stream."""
+3DMatch loader, collate layout, size bucketing, read-ahead stream.  What the unmodified reference computed or
+shipped is read from tests/golden/data.npz (tests/golden/make_golden.py:data_fixture)."""
 import os
 import pickle
 import sys
@@ -8,25 +9,20 @@ import numpy as np
 import pytest
 import torch
 
-from regtr_b200 import data as D
+from conftest import GOLDEN, REAL_CASES, load_golden, sha256_of
 
-REF = '/root/reference'
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
+import eval_inputs as ei  # noqa: E402
+from regtr_b200 import data as D  # noqa: E402
+
+
+@pytest.fixture(scope='module')
+def fx():
+    return load_golden('data')
 
 
 def _make_dataset(tmp_path, n_pairs=11, seed=0):
-    rng = np.random.default_rng(seed)
-    infos = dict(rot=[], trans=[], src=[], tgt=[], overlap=[])
-    os.makedirs(tmp_path / 'test' / 'scene', exist_ok=True)
-    for i in range(n_pairs + 1):
-        pts = rng.normal(size=(int(rng.integers(50, 400)), 3))                      # float64, like the real files
-        torch.save(pts, tmp_path / 'test' / 'scene' / f'cloud_bin_{i}.pth')
-    for i in range(n_pairs):
-        q, _ = np.linalg.qr(rng.normal(size=(3, 3)))
-        infos['rot'].append(q); infos['trans'].append(rng.normal(size=(3, 1)))
-        infos['src'].append(f'test/scene/cloud_bin_{i + 1}.pth'); infos['tgt'].append(f'test/scene/cloud_bin_{i}.pth')
-        infos['overlap'].append(float(rng.uniform(0.1, 0.9)))
-    with open(tmp_path / 'info.pkl', 'wb') as f:
-        pickle.dump(infos, f)
+    infos = ei.write_pair_files(str(tmp_path), n_pairs, seed)
     return D.ThreeDMatchPairs(str(tmp_path), str(tmp_path / 'info.pkl')), infos
 
 
@@ -43,33 +39,43 @@ def test_dataset_items_and_collate(tmp_path):
     assert b['overlap_p'].shape == (3,) and b['idx'] == [0, 1, 2]
 
 
-def test_collate_matches_reference_function(tmp_path):
-    if not os.path.isdir(REF):
-        pytest.skip('reference not present on this machine')
-    import importlib.util                       # the file only imports torch; its package __init__ needs h5py
-    spec = importlib.util.spec_from_file_location('ref_collate_functions',
-                                                  os.path.join(REF, 'src', 'data_loaders', 'collate_functions.py'))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    ref_collate = mod.collate_pair
+def test_collate_matches_reference_function(tmp_path, fx):
+    """collate_pair vs what the reference's data_loaders/collate_functions.py returned for the same three items."""
     ds, _ = _make_dataset(tmp_path)
     items = [ds[i] for i in (4, 0, 7)]
-    a, b = D.collate_pair(items), ref_collate(items)
-    assert set(a) == set(b)
+    a = D.collate_pair(items)
+    assert set(a) == set(fx['collate_keys'].tolist())
     for k in a:
         if torch.is_tensor(a[k]):
-            assert torch.equal(a[k], b[k])
+            want = fx[f'collate|{k}']
+            assert a[k].dtype == torch.from_numpy(want).dtype and torch.equal(a[k], torch.from_numpy(want))
         else:
-            assert len(a[k]) == len(b[k]) and all(
-                (torch.equal(x, y) if torch.is_tensor(x) else x == y) for x, y in zip(a[k], b[k]))
+            want = [fx[f'collate|{k}|{b}'] for b in range(sum(key.startswith(f'collate|{k}|') for key in fx))]
+            assert len(a[k]) == len(want) and all(
+                (torch.equal(x, torch.from_numpy(y)) if torch.is_tensor(x) else x == y.item()) for x, y in zip(a[k], want))
 
 
-def test_reads_the_reference_sample_pairs():
-    """The 3DMatch pairs shipped with the reference (data/indoor, demo.py) through the real benchmark pickle."""
-    root, info = os.path.join(REF, 'data', 'indoor'), os.path.join(REF, 'src', 'datasets', '3dmatch', 'test_3DMatch_info.pkl')
-    if not (os.path.isdir(root) and os.path.isfile(info)):
-        pytest.skip('reference data not present on this machine')
-    ds = D.ThreeDMatchPairs(root, info)
+def test_reads_the_reference_sample_pairs(tmp_path, fx):
+    """The 3DMatch pairs shipped with the reference (data/indoor, demo.py) through the real benchmark pickle, both
+    rebuilt from the fixtures: every row of test_3DMatch_info.pkl with the original Python types, and the clouds as
+    float64 files from the fp32 input fixtures (the shipped files hold fp32 values; their SHA-256 pins that)."""
+    root, info = tmp_path / 'indoor', tmp_path / 'test_3DMatch_info.pkl'
+    with open(info, 'wb') as f:
+        pickle.dump(dict(rot=list(fx['info_rot']), trans=list(fx['info_trans']), src=fx['info_src'].tolist(),
+                         tgt=fx['info_tgt'].tolist(), overlap=[np.float64(v) for v in fx['info_overlap']]), f)
+    n_clouds = 0
+    for case in REAL_CASES:
+        inp = np.load(os.path.join(GOLDEN, 'real', case + '_input.npz'))
+        for side in ('src', 'tgt'):
+            rel = str(inp[f'{side}_file'])
+            if rel.startswith('indoor/'):
+                cloud = inp[f'{side}_xyz'].astype(np.float64)
+                assert np.array_equal(sha256_of(cloud), fx[f'cloud_sha256|{rel}']), rel
+                os.makedirs(os.path.dirname(tmp_path / rel), exist_ok=True)
+                torch.save(cloud, tmp_path / rel)
+                n_clouds += 1
+    assert n_clouds == sum(k.startswith('cloud_sha256|') for k in fx) == 6
+    ds = D.ThreeDMatchPairs(str(root), str(info))
     assert len(ds) == 1623
     have = [i for i in range(len(ds)) if all(os.path.isfile(os.path.join(root, ds.infos[k][i])) for k in ('src', 'tgt'))]
     assert have, 'no complete pair among the shipped sample clouds'
@@ -104,12 +110,10 @@ def test_pair_stream_order_and_errors(tmp_path):
         list(D.PairStream(ds, batches, workers=2, depth=2))
 
 
-def test_sequence_helpers_match_reference():
-    """regtr_b200.seq vs utils/seq_manipulation.py (imported when the reference is present), plus a padded
-    round trip."""
+def test_sequence_helpers_match_reference(fx):
+    """regtr_b200.seq vs what utils/seq_manipulation.py returned on the same inputs, plus a padded round trip."""
     from regtr_b200 import seq as S
-    rng = np.random.default_rng(2)
-    seqs = [torch.from_numpy(rng.normal(size=(n, 5)).astype(np.float32)) for n in (7, 3, 11, 1)]
+    seqs, six = ei.seq_inputs()
     padded, mask, lens = S.pad_sequence(seqs, require_padding_mask=True, require_lens=True)
     assert padded.shape == (11, 4, 5) and mask.shape == (4, 11) and lens == [7, 3, 11, 1]
     assert mask[1, 3:].all() and not mask[1, :3].any() and not mask[2].any()
@@ -118,20 +122,17 @@ def test_sequence_helpers_match_reference():
     stacked = torch.cat(seqs)
     src, tgt = S.split_src_tgt(stacked, torch.tensor(lens))
     assert len(src) == 2 and torch.equal(tgt[1], seqs[3])
-    if os.path.isdir(REF):
-        import importlib.util
-        spec = importlib.util.spec_from_file_location('ref_seq', os.path.join(REF, 'src', 'utils', 'seq_manipulation.py'))
-        R = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(R)
-        for kw in (dict(), dict(require_padding_mask=True, require_lens=True)):
-            a, b = S.pad_sequence(seqs, **kw), R.pad_sequence(seqs, **kw)
-            assert torch.equal(a[0], b[0]) and (a[1] is None) == (b[1] is None) and a[2] == b[2]
-            if a[1] is not None:
-                assert torch.equal(a[1], b[1])
-        six = torch.from_numpy(rng.normal(size=(6, 11, 4, 5)).astype(np.float32))
-        assert all(torch.equal(x, y) for x, y in zip(S.unpad_sequences(six, lens), R.unpad_sequences(six, lens)))
-        a, b = S.split_src_tgt(stacked, lens), R.split_src_tgt(stacked, lens)
-        assert all(torch.equal(x, y) for x, y in zip(a[0] + a[1], b[0] + b[1]))
+    T = lambda key: torch.from_numpy(fx[key])
+    for i, kw in enumerate((dict(), dict(require_padding_mask=True, require_lens=True))):
+        a = S.pad_sequence(seqs, **kw)
+        assert torch.equal(a[0], T(f'pad{i}_padded'))
+        assert (a[1] is None) == (f'pad{i}_mask' not in fx) and (a[2] is None) == (f'pad{i}_lens' not in fx)
+        if a[1] is not None:
+            assert torch.equal(a[1], T(f'pad{i}_mask')) and a[2] == fx[f'pad{i}_lens'].tolist()
+    got = S.unpad_sequences(six, lens)
+    assert len(got) == 4 and all(torch.equal(x, T(f'unpad_{b}')) for b, x in enumerate(got))
+    a = S.split_src_tgt(stacked, lens)
+    assert len(a[0]) == len(a[1]) == 2 and all(torch.equal(x, T(f'split_{b}')) for b, x in enumerate(a[0] + a[1]))
 
 
 def test_compute_overlap_properties(tmp_path):
